@@ -103,6 +103,25 @@ def note(msg: str):
     print(f"[bench {time.strftime('%H:%M:%S')}] {msg}", file=sys.stderr, flush=True)
 
 
+def dump_outputs(out_dir, calls):
+    """--dump-outputs: what the last timed step returned to its caller, one policy() call after the other, as float npy files:
+    wav (every emitted waveform chunk, concatenated), write and samples_per_call (the action and chunk length of each call), and the
+    latest asr_tokens / st_tokens / mt_tokens / units / dur of the step (the complete hypotheses of the utterance)."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    wavs = [wav.float().cpu().numpy() for w, wav, _ in calls if w and wav is not None]
+    arrays = {"wav": np.concatenate(wavs) if wavs else np.zeros(0, dtype=np.float32),
+              "write": np.array([float(w) for w, _, _ in calls]),
+              "samples_per_call": np.array([float(wav.numel()) if w and wav is not None else 0.0 for w, wav, _ in calls])}
+    for key in ("asr_tokens", "st_tokens", "mt_tokens", "units", "dur"):
+        seen = [tr[key] for _, _, tr in calls if key in tr]
+        arrays[key] = np.array(seen[-1] if seen else [], dtype=np.float64)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+    return sum(a.nbytes for a in arrays.values())
+
+
 def run_reference(args):
     """CPU arm: the reference agent's semantics (full-prefix recompute every chunk) in PyTorch fp32 on the host cores."""
     import torch
@@ -420,6 +439,8 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip the configs[2] / configs[3] legs (extra keys of the JSON line)")
     ap.add_argument("--ncu-window", action="store_true",
                     help="after the timed runs, stream one more resident utterance between cudaProfilerStart/Stop (for `ncu --profile-from-start off`)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (waveform, actions, tokens) as DIR/<name>.npy, to compare two builds")
     args = ap.parse_args()
     if args.impl == "reference":
         return run_reference(args)
@@ -482,7 +503,7 @@ def main():
     utts_dev = [u.cuda() for u in utts]
     flush = torch.empty(256 * 1024 * 1024 // 4, dtype=torch.float32, device="cuda")  # > 126 MB L2
 
-    def stream_resident(u):
+    def stream_resident(u, calls=None):
         agent.reset()
         out = 0
         for i in range(0, u.numel(), n):
@@ -490,6 +511,8 @@ def main():
             w, wav = agent.step_resident(u, end, end >= u.numel())
             if w and wav is not None:
                 out += wav.numel()
+            if calls is not None:  # every call returns a fresh wav tensor and trace dict: keeping them costs no device work
+                calls.append((w, wav, agent.trace))
         return out
 
     def stream_e2e(u_host):
@@ -501,7 +524,7 @@ def main():
                 out += len(seg.content)
         return out
 
-    def timed(fn, inputs, steps, warmup):
+    def timed(fn, inputs, steps, warmup, last_calls=None):
         for i in range(warmup):
             fn(inputs[i % len(inputs)])
         if dist is not None:
@@ -510,10 +533,11 @@ def main():
         total_ms, out = 0.0, 0
         l0 = eng.launch_count()
         for i in range(steps):
+            record = (last_calls,) if last_calls is not None and i == steps - 1 else ()
             flush.fill_(float(i))  # L2 flush between timed iterations (outside the events)
             s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             s.record()
-            out += fn(inputs[i % len(inputs)])
+            out += fn(inputs[i % len(inputs)], *record)
             e.record()
             torch.cuda.synchronize()
             total_ms += s.elapsed_time(e)
@@ -528,7 +552,12 @@ def main():
     if rank == 0:
         sampler.start()
     note("timed: resident")
-    ms_res, out_res, launches = timed(stream_resident, utts_dev, args.steps, args.warmup)
+    last_calls = [] if args.dump_outputs and rank == 0 else None
+    ms_res, out_res, launches = timed(stream_resident, utts_dev, args.steps, args.warmup, last_calls)
+    if last_calls is not None:
+        nbytes = dump_outputs(args.dump_outputs, last_calls)
+        note(f"outputs of the last timed step: {len(last_calls)} calls, {nbytes} bytes -> {args.dump_outputs}")
+        del last_calls
     note("timed: e2e")
     utts_host = [u.tolist() for u in utts]
     ms_e2e, out_e2e, _ = timed(stream_e2e, utts_host, args.steps, max(1, args.warmup // 2))

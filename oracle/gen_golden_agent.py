@@ -16,7 +16,7 @@ A1.  `StreamSpeechS2STAgent.policy` and `.reset` (agent:328-347,422-770) and `On
      are streamed; `OracleS2STAgent` must reproduce every action: READ / WRITE, the flags, token sequences, units, durations and
      the waveform.
 
-Both write fixtures to tests/golden/ (mt_greedy.npz, agent_policy.npz) that the CPU tests replay against the oracle and the
+Both write fixtures to tests/golden/ (mt_greedy.npz, agent_policy_<tag>.npz) that the CPU tests replay against the oracle and the
 GPU tests against the engine.
 """
 from __future__ import annotations
@@ -361,13 +361,12 @@ def main():
     gcmvn = synth.make_gcmvn(cfg)
     report = {}
     pin_mt_greedy(cfg, sd, gcmvn, report)
-    out = {}
+    # one file per utterance keeps every fixture file under 1 MB
     for tag, seg_ms, seconds, seed in (("c320", 320, 3.2, 1234), ("c640", 640, 3.84, 1234)):
         r = run_policy_pair(cfg, sd, vsd_wn, gcmvn, seg_ms, seconds, seed, report, tag)
-        out.update({f"{tag}_{k}": v for k, v in r.items()})
+        np.savez_compressed(os.path.join(GOLD, f"agent_policy_{tag}.npz"), **{f"{tag}_{k}": v for k, v in r.items()})
     r = run_s2tt_pair(cfg, sd, gcmvn, 320, 2.56, 1234, report, "s2tt320")
-    out.update({f"s2tt320_{k}": v for k, v in r.items()})
-    np.savez_compressed(os.path.join(GOLD, "agent_policy.npz"), **out)
+    np.savez_compressed(os.path.join(GOLD, "agent_policy_s2tt320.npz"), **{f"s2tt320_{k}": v for k, v in r.items()})
     for k, v in report.items():
         print(f"{k:28s} {v}")
 

@@ -500,13 +500,13 @@ def test_mt_greedy_reference_generate_decoder_fixture(full, gold):
 
 @pytest.mark.parametrize("tag", ["c320", "c640"])
 def test_s2st_agent_vs_reference_policy_fixture(gold, tag):
-    """A1 / P1 against the REAL reference: tests/golden/agent_policy.npz is the action sequence of the reference's own policy()
+    """A1 / P1 against the REAL reference: tests/golden/agent_policy_<tag>.npz is the action sequence of the reference's own policy()
     (agent:422-770, executed from its source on reference generator / module objects, oracle/gen_golden_agent.py).  The engine
     agent must take the same READ / WRITE decisions, emit the same units and the same waveform (1e-3)."""
     from streamspeech_b200.agent import StreamSpeechS2STAgent
     from streamspeech_b200.simuleval_compat import SpeechSegment
 
-    g = gold["agent_policy"]
+    g = gold[f"agent_policy_{tag}"]
     seg_ms, seconds, seed = int(g[f"{tag}_segment_ms"]), float(g[f"{tag}_seconds"]), int(g[f"{tag}_seed"])
     agent = StreamSpeechS2STAgent(agent_args(source_segment_size=seg_ms))
     wav = synth.make_audio(seconds, seed=seed)
@@ -533,15 +533,15 @@ def test_s2st_agent_vs_reference_policy_fixture(gold, tag):
 
 def test_s2tt_agent_vs_reference_policy_fixture_and_oracle(gold):
     """Row f1: StreamSpeechS2TTAgent (incremental MT decoder states across policy() calls, SURVEY.md N12) against (a) the action
-    sequence of the reference's own S2TT policy() (tests/golden/agent_policy.npz, oracle/gen_golden_agent.py) and (b) the oracle
-    agent on a second utterance: every text delta and every hypothesis bit-exact."""
+    sequence of the reference's own S2TT policy() (tests/golden/agent_policy_s2tt320.npz, oracle/gen_golden_agent.py) and (b) the
+    oracle agent on a second utterance: every text delta and every hypothesis bit-exact."""
     from oracle.agent_oracle import OracleS2TTAgent
     from oracle.streamspeech_oracle import StreamSpeechOracle
     from streamspeech_b200.agent import StreamSpeechS2TTAgent
     from streamspeech_b200.dictionary import Dictionary
     from streamspeech_b200.simuleval_compat import SpeechSegment
 
-    g = gold["agent_policy"]
+    g = gold["agent_policy_s2tt320"]
     tag = "s2tt320"
     seg_ms, seconds, seed = int(g[f"{tag}_segment_ms"]), float(g[f"{tag}_seconds"]), int(g[f"{tag}_seed"])
     agent = StreamSpeechS2TTAgent(agent_args(source_segment_size=seg_ms))

@@ -194,13 +194,13 @@ def test_mt_greedy_matches_reference_generate_decoder(gold):
 
 @pytest.mark.parametrize("tag", ["c320", "c640"])
 def test_agent_oracle_matches_reference_policy_fixture(gold, tag):
-    """A1 / P1 pin: tests/golden/agent_policy.npz is the action sequence of the reference's own `policy()` (executed from its
+    """A1 / P1 pin: tests/golden/agent_policy_<tag>.npz is the action sequence of the reference's own `policy()` (executed from its
     source on reference generator / module objects, oracle/gen_golden_agent.py) for a 320 ms utterance and a 640 ms
     (whole-word, agent:540-574) utterance.  OracleS2STAgent must reproduce every READ / WRITE, the flags, and the waveform."""
     from oracle.agent_oracle import OracleS2STAgent
     from streamspeech_b200.dictionary import Dictionary
 
-    g = gold["agent_policy"]
+    g = gold[f"agent_policy_{tag}"]
     cfg = ModelConfig()
     o = StreamSpeechOracle(cfg, synth.make_model_state_dict(cfg, 0), synth.make_vocoder_state_dict(cfg.vocoder, 1, weight_norm=True),
                            synth.make_gcmvn(cfg))
@@ -231,7 +231,7 @@ def test_s2tt_oracle_matches_reference_policy_fixture(gold):
     from oracle.agent_oracle import OracleS2TTAgent
     from streamspeech_b200.dictionary import Dictionary
 
-    g = gold["agent_policy"]
+    g = gold["agent_policy_s2tt320"]
     cfg = ModelConfig()
     o = StreamSpeechOracle(cfg, synth.make_model_state_dict(cfg, 0), None, synth.make_gcmvn(cfg))
     d = Dictionary.synthetic(cfg.tgt_vocab)
